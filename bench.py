@@ -307,9 +307,30 @@ def emit(line):
         os.write(_JSON_FD, data)
 
 
-def measure(args, n, bits, plc, loss, hops, warm_hops, kernel_hops, e2e_hops, world, rank, local_rank, decoder_mode, want_clocks):
+DUMP_MAX_BYTES = 63 * 10 ** 6      # --dump-outputs: all arrays together stay under 64 MB, .npy headers included
+
+
+def write_outputs(out_dir, outputs):
+    """--dump-outputs: every array (one row per stream) as float32 DIR/<name>.npy.  When they would exceed DUMP_MAX_BYTES
+    together, every array keeps the same fixed, seeded sample of stream rows (in stream order).  Returns the rows kept."""
+    import numpy as np
+    n = len(next(iter(outputs.values())))
+    row_bytes = sum(4 * (a.size // n) for a in outputs.values())
+    rows = np.arange(n)
+    if n * row_bytes > DUMP_MAX_BYTES:
+        rows = np.sort(np.random.default_rng(SEED).choice(n, DUMP_MAX_BYTES // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a)[rows].astype(np.float32))
+    return rows
+
+
+def measure(args, n, bits, plc, loss, hops, warm_hops, kernel_hops, e2e_hops, world, rank, local_rank, decoder_mode, want_clocks,
+            dump=False):
     """One configuration on this rank's GPU: device-resident throughput over `hops` hops, a serialised per-kernel pass, and the
-    end-to-end pass through the host-buffer C ABI.  Returns a dict; multi-rank reductions (max over ranks) are done inside."""
+    end-to-end pass through the host-buffer C ABI.  Returns a dict; multi-rank reductions (max over ranks) are done inside.
+    dump: the result's "outputs" holds what each timed pass returned for the last hop it timed (decoded PCM, and the packets or,
+    for the decoder-only workload, the comfort-noise flags), one row per stream."""
     import ctypes as C
     import numpy as np
     import torch
@@ -449,6 +470,13 @@ def measure(args, n, bits, plc, loss, hops, warm_hops, kernel_hops, e2e_hops, wo
     clocks = sampler.stop() if sampler else None
     gpu_launches = sum(c.launch_count for c in group_ctxs) - launches0
     barrier()
+    outputs = {}
+    if dump:     # read before the per-kernel pass below reuses the buffers
+        outputs["pcm"] = d_out.cpu().numpy()
+        if plc:
+            outputs["is_comfort_noise"] = d_flags.cpu().numpy()
+        else:
+            outputs["packets"] = d_pks[(hops - 1) % NBUF].cpu().numpy()
     # per-kernel roofline pass on the full-size context pair: the same hops with the kernels serialised (one launch per kernel
     # and hop over all n streams, no concurrent sub-batches, no encode/decode overlap), CUDA events around every launch
     full = [(enc, dec, sx, sy)]
@@ -562,6 +590,12 @@ def measure(args, n, bits, plc, loss, hops, warm_hops, kernel_hops, e2e_hops, wo
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     e2e_value = world * n * e2e_hops / float(t.item())
+    if dump:
+        outputs["e2e_pcm"] = pin_out.numpy().copy()
+        if plc:
+            outputs["e2e_is_comfort_noise"] = pin_flags.numpy().copy()
+        else:
+            outputs["e2e_packets"] = pin_pks[(e2e_hops - 1) % NBUF].numpy().copy()
     checksum = int(pin_out.to(torch.int64).sum().item())
     tile_streams = dec.tile_streams
     graph_replays = sum(c.graph_replays() for c in host_ctxs)
@@ -569,7 +603,7 @@ def measure(args, n, bits, plc, loss, hops, warm_hops, kernel_hops, e2e_hops, wo
         c.close()
     return {"value": value, "elapsed_ms": elapsed_ms, "e2e_value": e2e_value, "e2e_s": float(t.item()), "prof": prof, "clocks": clocks,
             "gpu_launches": int(gpu_launches), "checksum": checksum, "G": G, "Gh": Gh, "oversubscribed": oversubscribed, "tile_streams": tile_streams, "stream_priority": {"device_pass": {"encoder": prio_x, "decoder": prio_y}, "host_pass": {"encoder": host_prio_x, "decoder": host_prio_y}},
-            "P": P, "graph_replays": graph_replays}
+            "P": P, "graph_replays": graph_replays, "outputs": outputs}
 
 
 def roofline_of(res, n, bits, plc, world, hops, decoder_mode, clocks):
@@ -639,6 +673,11 @@ def main():
     ap.add_argument("--decoder-mode", default="tensor", choices=["exact", "tensor"],
                     help="tensor (default): the decoder's fp32 GEMMs on the tensor cores (kernel D: tcgen05 UMMA), decoded PCM within "
                          "4 int16 LSB of the oracle, packets bit-exact; exact: decoded PCM bit-identical to the oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed passes returned for their last hop as DIR/<name>.npy (float32, "
+                         "one row per stream; pcm and packets, or is_comfort_noise for decode_plc; e2e_* from the host-buffer pass), "
+                         "under 64 MB in all (a fixed, seeded sample of the streams when larger).  The inputs depend only on the "
+                         "arguments, so two builds can be compared output for output")
     args = ap.parse_args()
     if args.bits is None:
         args.bits = 120 if args.gpus >= 8 else 64
@@ -664,9 +703,14 @@ def main():
     n, bits = args.streams, args.bits
     plc = args.workload == "decode_plc"
     hops = args.steps * HOPS_PER_STEP
+    dump = args.dump_outputs is not None and rank == 0
     res = measure(args, n, bits, plc, args.loss, hops, max(3, args.warmup) * HOPS_PER_STEP, min(hops, 40), hops, world, rank, local_rank,
-                  args.decoder_mode, want_clocks=True)
+                  args.decoder_mode, want_clocks=True, dump=dump)
     value, e2e_value, clocks, P, G = res["value"], res["e2e_value"], res["clocks"], res["P"], res["G"]
+    if dump:
+        rows = write_outputs(args.dump_outputs, res["outputs"])
+        print("bench.py: wrote %s (%d of %d streams) to %s" % (", ".join(sorted(res["outputs"])), len(rows), n, args.dump_outputs),
+              file=sys.stderr)
 
     other = None
     if world == 1 and not args.no_other_configs and not plc:

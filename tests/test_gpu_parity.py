@@ -347,13 +347,12 @@ def test_umma_probes_on_hardware(tmp_path, probe, cases):
     """tests/cpp/umma_probe{,2}.cu built with nvcc: the tcgen05 / TMEM instruction sequences of device_compat.h that the product's
     UMMA kernel (DecoderKernelDU) is made of - shared-memory descriptors, split-precision TF32 MMAs, A operands in tensor memory,
     tcgen05.st / wide tcgen05.ld, kind::i8, N = 160 / 16 shapes, bulk stores.  The product depends on them: a mismatch is a failure."""
-    import shutil
     import subprocess
+
+    import __graft_entry__ as g
     from conftest import ROOT
-    if shutil.which("nvcc") is None:
-        pytest.skip("nvcc not available on this box")
     exe = str(tmp_path / probe)
-    subprocess.check_call(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-I" + os.path.join(ROOT, "lyra_b200", "csrc"),
+    subprocess.check_call([g.NVCC, "-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-I" + os.path.join(ROOT, "lyra_b200", "csrc"),
                            "-o", exe, os.path.join(ROOT, "tests", "cpp", probe + ".cu")])
     out = subprocess.run(["timeout", "60", exe], capture_output=True, text=True, timeout=120)
     print(out.stdout.strip())

@@ -89,3 +89,28 @@ def test_bench_host_pass_groups():
     assert bench.host_pass_priorities(2, 64, False) == (0, 0)
     assert bench.host_pass_priorities(2, 120, False) == (-1, 0)      # two groups, long RVQ chains: encoder first
     assert bench.host_pass_priorities(2, 184, True) == (0, 0)        # decoder-only workload
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 .npy files, every stream while they fit the budget, else the same seeded rows of each."""
+    sys.path.insert(0, ROOT)
+    import bench
+    n = 1000
+    pcm = np.arange(n * 320, dtype=np.int64).reshape(n, 320).astype(np.int16)
+    outputs = {"pcm": pcm, "packets": (np.arange(n * 8) % 256).astype(np.uint8).reshape(n, 8)}
+    rows = bench.write_outputs(str(tmp_path / "all"), outputs)
+    assert rows.tolist() == list(range(n))
+    for name, a in outputs.items():
+        got = np.load(str(tmp_path / "all" / (name + ".npy")))
+        assert got.dtype == np.float32 and np.array_equal(got, a.astype(np.float32))
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 100 * (320 + 8) * 4)
+    rows = bench.write_outputs(str(tmp_path / "a"), outputs)
+    assert len(rows) == 100 and (np.diff(rows) > 0).all()
+    assert np.array_equal(rows, bench.write_outputs(str(tmp_path / "b"), outputs))
+    total = 0
+    for name, a in outputs.items():
+        got = np.load(str(tmp_path / "a" / (name + ".npy")))
+        assert np.array_equal(got, a[rows].astype(np.float32))
+        assert np.array_equal(got, np.load(str(tmp_path / "b" / (name + ".npy"))))
+        total += got.nbytes
+    assert total <= bench.DUMP_MAX_BYTES
