@@ -10,7 +10,9 @@
 //               its other lanes hold stale data, which only reaches accumulator rows nobody reads - GEMM rows are independent).
 //   residual    A operand in TENSOR MEMORY, written by the row's own thread with tcgen05.st (hi and lo column blocks): the
 //   units       activations never take a round trip through shared memory between the depthwise conv, the two 1x1 convolutions
-//               and last_layer.  B = weights from shared memory.
+//               and last_layer.  B = weights from shared memory.  The A operand is staged one k-half (32 channels) at a time in
+//               the same 64 columns: the row warps write channels 32..63 once the MMAs that read 0..31 have completed (a_free).
+//               With D that is 128 columns per row block, 256 per tile: two blocks share the SM's tensor memory.
 //   decoder_2/  computed TRANSPOSED: the 640 weight rows (tap j, phase r, cout) are the M dimension (five 128-row blocks, A operand
 //   simple      from shared memory) and the tile's 32 (input row, stream) pairs the N dimension (B operand, 16 KB per half): a
 //               16-cycle MMA instead of an 80-cycle one whose 128 rows would be three-quarters padding, and an epilogue in
@@ -62,8 +64,8 @@ struct DecDU {
   static constexpr int kDw4 = kSlOut + 48 * S * 4;            // depthwise parameters per channel: float4 {w0, w1, w2, bias} [3][64]
   static constexpr int kW = kDw4 + 3 * 256 * 4;               // weight ring
   static constexpr int kI = kW + kStagesW * kDuChunkBytes;    // slot[S], active[S], n18[S]
-  // LYRA_DU_SMEM_PAD: request more than the layout needs, e.g. 6144 -> 116 KB = at most one block of this kernel per SM (the second
-  // resident block waits for tensor memory most of its life while holding 110 KB that a kernel-A / B / C block could use)
+  // LYRA_DU_SMEM_PAD: request more than the layout needs, e.g. 6144 -> 116 KB = at most one block of this kernel per SM (the rest of
+  // the SM is left to a kernel-A / B / C block)
 #ifndef LYRA_DU_SMEM_PAD
 #define LYRA_DU_SMEM_PAD 0
 #endif
@@ -72,9 +74,11 @@ struct DecDU {
   static_assert(kXc % 128 == 0 && kOv % 128 == 0 && kRing0 % 128 == 0 && kRing1 % 128 == 0 && kW % 128 == 0 && kSl % 16 == 0 && kDw4 % 16 == 0,
                 "bulk-copy / descriptor alignment");
   static_assert(kSmemBytes - LYRA_DU_SMEM_PAD <= 113 * 1024, "must leave room for a kernel-A block on the SM");
-  // tensor memory columns (512 allocated).  decoder_2/simple: block mb at columns 32 mb.  Afterwards per row block rb: A hi | A lo | D
-  static constexpr int kTmemCols = 512;
-  static constexpr int kColAhi = 0, kColAlo = 64, kColD = 128, kRbStride = 192;
+  // tensor memory columns: 256, half of the SM's, so that two blocks of this kernel run at once.  decoder_2/simple: block mb at
+  // columns 32 mb.  Afterwards per row block rb: A hi | A lo of ONE k-half (channels 0..31, then 32..63 in the same columns) | D
+  static constexpr int kTmemCols = 256;
+  static constexpr int kColAhi = 0, kColAlo = 32, kColD = 64, kRbStride = 128;
+  static_assert(5 * 32 <= kTmemCols && 2 * kRbStride <= kTmemCols, "decoder_2/simple's accumulators and both row blocks fit");
 };
 
 struct DecDUShared {
@@ -83,7 +87,8 @@ struct DecDUShared {
   LyraMbar s_full[DecDU::kStagesW];     // row warps -> MMA issuer: the chunk is split (hi | lo) in place
   LyraMbar in_full;        // producer -> row warps: the last_layer tail has landed
   LyraMbar ov_full;        // producer -> row warps: the overlap tail has landed (in the X region, after decoder_2/simple's MMAs)
-  LyraMbar a_ready;        // row warps -> MMA issuer: the operand of the next GEMM is in place
+  LyraMbar a_ready;        // row warps -> MMA issuer: the operand of the next GEMM (or k-half of it) is in place
+  LyraMbar a_free;         // MMA issuer -> row warps: the MMAs that read the A operand's first k-half have completed
   LyraMbar d_ready;        // MMA issuer -> row warps: the accumulators of the GEMM are complete
   LyraMbar ring_full[2];   // producer -> row warps: ring block u (units 0, 1) has landed
   LyraMbar tmem_ready;     // MMA warp -> everybody: tensor memory is allocated, tmem_base is valid
@@ -127,7 +132,67 @@ __device__ __forceinline__ void DuForEachAccGroup(uint32_t taddr, F f) {
   }
 }
 
-__global__ void __launch_bounds__(DecDU::NT, 1)
+// All row threads: between the two k-halves of an A operand, wait until the MMAs that read the first half have completed.
+__device__ __forceinline__ void DuWaitAFree(DecDUShared* sh, unsigned& par) {
+  lyra_mbar_wait(&sh->a_free, par);
+  par ^= 1;
+  lyra_tc_fence_after_sync();
+}
+
+// All row threads: the next GEMM's A operand, 16 channels at a time, make(c0, hi, lo) for c0 = 0, 16 | 32, 48, written to
+// the row's A columns in two k-halves: channels 0..31 are published, then 32..63 overwrite them once the MMAs that read the
+// first half have completed.
+template <typename F>
+__device__ __forceinline__ void DuWriteA(DecDUShared* sh, uint32_t trow, bool has_row, unsigned& f_par, F make) {
+#pragma unroll 1
+  for (int h = 0; h < 2; ++h) {
+    if (h == 1) DuWaitAFree(sh, f_par);
+    if (has_row) {
+#pragma unroll 1
+      for (int c0 = 32 * h; c0 < 32 * h + 32; c0 += 16) {
+        uint32_t hi[16], lo[16];
+        make(c0, hi, lo);
+        lyra_tmem_st<16>(trow + DecDU::kColAhi + (uint32_t)(c0 - 32 * h), hi);
+        lyra_tmem_st<16>(trow + DecDU::kColAlo + (uint32_t)(c0 - 32 * h), lo);
+      }
+    }
+    DuArriveA(sh);
+  }
+}
+
+// All row threads: the GEMM's accumulators (64 columns at trow + kColD) -> the next GEMM's A operand in two k-halves,
+// f(c0, v, hi, lo) converting 16 channels.  The next GEMM's first MMAs overwrite D, so columns 32..63 are loaded into
+// registers before the first half is published and converted after a_free.  Warp-collective.
+template <typename F>
+__device__ __forceinline__ void DuAccToA(DecDUShared* sh, uint32_t trow, bool has_row, unsigned& f_par, F f) {
+  uint32_t v[2][16];
+  auto put = [&](int c0, const uint32_t (&x)[16]) {
+    uint32_t hi[16], lo[16];
+    f(c0, x, hi, lo);
+    lyra_tmem_st<16>(trow + DecDU::kColAhi + (uint32_t)(c0 % 32), hi);
+    lyra_tmem_st<16>(trow + DecDU::kColAlo + (uint32_t)(c0 % 32), lo);
+  };
+  if (has_row) {
+    const uint32_t td = trow + DecDU::kColD;
+    lyra_tmem_ld<16>(td, v[0]);
+    lyra_tmem_wait_ld();
+    lyra_tmem_ld<16>(td + 16u, v[1]);
+    put(0, v[0]);
+    lyra_tmem_wait_ld();
+    lyra_tmem_ld<16>(td + 32u, v[0]);
+    put(16, v[1]);
+    lyra_tmem_ld<16>(td + 48u, v[1]);
+  }
+  DuArriveA(sh);                                             // (waits for the loads: D is read in full)
+  DuWaitAFree(sh, f_par);
+  if (has_row) {
+    put(32, v[0]);
+    put(48, v[1]);
+  }
+  DuArriveA(sh);
+}
+
+__global__ void __launch_bounds__(DecDU::NT, 2)
 DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, const float* __restrict__ mid,
                 float* __restrict__ state, int* __restrict__ n18g, int16_t* __restrict__ pcm, int ntiles) {
   using L = DecDU;
@@ -176,6 +241,7 @@ DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, co
     lyra_mbar_init(&sh->tmem_ready, 1);
     lyra_mbar_init(&sh->tmem_done, 5);
     lyra_mbar_init(&sh->a_ready, L::kRowWarps);
+    lyra_mbar_init(&sh->a_free, 1);
     lyra_mbar_init(&sh->d_ready, 1);
     for (int i = 0; i < 2; ++i) lyra_mbar_init(&sh->ring_full[i], 1);
     lyra_mbar_fence_init();
@@ -188,10 +254,9 @@ DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, co
   int ph = 0;
   const bool idle = n18[S] == kTileIdle;
   if (!idle) PrefetchTileState<LYRA_PREFETCH_STATE>(st, DecStateD::kUnits * S * 4);      // unit 2 reads its ring block from global memory
-  // Tensor memory is taken AFTER the block barriers above, by the MMA warp alone.  Two blocks of this kernel fit on an SM (shared
-  // memory, registers) but each needs all 512 TMEM columns, so the second one blocks in tcgen05.alloc until the first has
-  // finished - meanwhile its other warps already stage everything that does not need tensor memory (tile metadata, the X
-  // operand, the first weight chunks, depthwise parameters): the next tile's prologue runs under the current tile's tail.
+  // Tensor memory is taken AFTER the block barriers above, by the MMA warp alone.  A block takes 256 of the SM's 512 columns, so
+  // the two blocks of this kernel that fit on an SM (shared memory, registers) run at once: one tile's latency-bound residual
+  // units overlap the other's stream-bound decoder_2/simple phase.
   if (!idle && warp == L::kMmaWarp) {
     lyra_tmem_alloc(&sh->tmem_base, L::kTmemCols);
     lyra_tc_fence_before_sync();
@@ -285,8 +350,8 @@ DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, co
         const uint32_t idesc = lyra_umma_idesc_tf32(128, 64);
         const uint32_t lboW = 8u * 128u;
         for (int g = 0; g < 7; ++g) {
-          wait_a();
-          for (int kc = 0; kc < 2; ++kc) {
+          for (int kc = 0; kc < 2; ++kc) {                   // k-half kc: channels 32 kc .. 32 kc + 31, in the same A columns for both
+            wait_a();
             const unsigned char* wst = wait_chunk();
 #pragma unroll
             for (int k4 = 0; k4 < 4; ++k4) {
@@ -299,11 +364,12 @@ DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, co
                 for (int rb = 0; rb < 2; ++rb) {             // alternate the two row blocks' accumulators: MMAs into one TMEM tile run as
                                                              // a dependent chain (measured 56 cycles each here), interleaved ones overlap (24)
                   const uint32_t base = tmem + (uint32_t)(rb * L::kRbStride);
-                  lyra_umma_tf32_ts(base + L::kColD, base + (term == 0 ? L::kColAlo : L::kColAhi) + (uint32_t)(8 * ks), term == 1 ? bl : bh, idesc,
+                  lyra_umma_tf32_ts(base + L::kColD, base + (term == 0 ? L::kColAlo : L::kColAhi) + (uint32_t)(8 * k4), term == 1 ? bl : bh, idesc,
                                     ks > 0 || term > 0);
                 }
             }
             release_chunk();
+            if (kc == 0) lyra_umma_commit(&sh->a_free);      // the row warps may overwrite the A columns with the second half
           }
           lyra_umma_commit(&sh->d_ready);
         }
@@ -311,7 +377,7 @@ DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, co
     }
 #if LYRA_DU_EARLY_DEALLOC
     // Tensor memory goes back as soon as the row warps have read the last accumulators - not at block exit, after the PCM and
-    // state stores - so that the next resident block's tcgen05.alloc returns that much earlier.
+    // state stores - so that a block that asks for it meanwhile does not wait for those stores.
     __syncwarp();
     lyra_mbar_wait(&sh->tmem_done, 0);
     lyra_tc_fence_after_sync();
@@ -325,7 +391,7 @@ DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, co
     const int t = row / S, s = row % S;
     const int rb = row / 128;
     const bool has_row = warp < 5;                           // whole warps: tcgen05.ld / st are warp-collective
-    unsigned d_par = 0;
+    unsigned d_par = 0, f_par = 0;
     LYRA_PHASE(3, ph);
     auto wait_d = [&]() { lyra_mbar_wait(&sh->d_ready, d_par); d_par ^= 1; lyra_tc_fence_after_sync(); };
     auto row_sync = [&]() { lyra_named_bar_sync(1, L::kRowThreads); };
@@ -439,9 +505,10 @@ DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, co
       const int base = (n18[s] * 20) % R;                    // ring slot of this frame's row 0 for this stream
       if (ring_in_smem) lyra_mbar_wait(&sh->ring_full[unit < 2 ? unit : 0], 0);
       LYRA_PHASE(3, ph);
-      // depthwise conv (k = 3, dilation dil) over LeakyReLU(u) -> A operand (hi, lo) of pw1.  Rows before this frame come from
-      // the ring (already activated): source pointer, channel stride and negative slope are selected once, the loop is branch-free
-      if (has_row) {
+      // depthwise conv (k = 3, dilation dil) over LeakyReLU(u) -> A operand (hi, lo) of pw1, in two k-halves.  Rows before this
+      // frame come from the ring (already activated): source pointer, channel stride and negative slope are selected once, the
+      // loop is branch-free
+      {
         const float4* w4 = reinterpret_cast<const float4*>(smf + L::kDw4 / 4) + unit * 64;      // per channel {w0, w1, w2, bias}
         const bool r1 = t - dil < 0, r0 = t - 2 * dil < 0;
         const float* p2 = u + row;
@@ -449,8 +516,7 @@ DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, co
         const float* p0 = r0 ? ringp + ((base + t - 2 * dil + 2 * R) % R) * S + s : u + row - 2 * dil * S;
         const int st1 = r1 ? R * S : LDU, st0 = r0 ? R * S : LDU;
         const float n1 = r1 ? 1.0f : 0.3f, n0 = r0 ? 1.0f : 0.3f;
-        for (int c0 = 0; c0 < 64; c0 += 16) {
-          uint32_t hi[16], lo[16];
+        DuWriteA(sh, trow, has_row, f_par, [&](int c0, uint32_t (&hi)[16], uint32_t (&lo)[16]) {
           float x1v[16], x0v[16];
 #pragma unroll
           for (int j = 0; j < 16; ++j) { x1v[j] = p1[(c0 + j) * st1]; x0v[j] = p0[(c0 + j) * st0]; }      // the (possibly global) loads first
@@ -467,11 +533,8 @@ DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, co
             acc = __fmaf_rn(x2, wc.z, acc);
             DuSplit(__fadd_rn(acc, wc.w), hi[j], lo[j]);
           }
-          lyra_tmem_st<16>(trow + L::kColAhi + (uint32_t)c0, hi);
-          lyra_tmem_st<16>(trow + L::kColAlo + (uint32_t)c0, lo);
-        }
+        });
       }
-      DuArriveA(sh);
       LYRA_PHASE(3, ph);
       // The newest min(20, R) rows of lrelu(u) replace the ring's oldest entries (every slot: R <= 20).  The copy runs in two
       // halves, each behind one of the unit's two GEMMs, so the row threads are busy while the tensor core works.
@@ -489,17 +552,13 @@ DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, co
       // pw1 epilogue: bias, LeakyReLU, split -> A operand of pw2 (same TMEM columns: pw1's MMAs have completed)
       wait_d();
       LYRA_PHASE(3, ph);
-      if (has_row) {
+      {
         const float* b1 = BlobPtr<float>(blob, p.pw1.bias);
-        DuForEachAccGroup(trow + L::kColD, [&](int c0, const uint32_t (&v)[16]) {
-          uint32_t hi[16], lo[16];
+        DuAccToA(sh, trow, has_row, f_par, [&](int c0, const uint32_t (&v)[16], uint32_t (&hi)[16], uint32_t (&lo)[16]) {
 #pragma unroll
           for (int j = 0; j < 16; ++j) DuSplit(LeakyRelu(__fadd_rn(__uint_as_float(v[j]), b1[c0 + j])), hi[j], lo[j]);
-          lyra_tmem_st<16>(trow + L::kColAhi + (uint32_t)c0, hi);
-          lyra_tmem_st<16>(trow + L::kColAlo + (uint32_t)c0, lo);
         });
       }
-      DuArriveA(sh);
       ring_update(32);
       lyra_fence_proxy_async();
       row_sync();
@@ -509,28 +568,30 @@ DecoderKernelDU(const uint8_t* __restrict__ blob, DecoderParams P, TileIo io, co
       // unit 2: LeakyReLU(u') straight into tensor memory as the A operand of last_layer
       wait_d();
       LYRA_PHASE(3, ph);
-      if (has_row) {
+      {
         const float* b2 = BlobPtr<float>(blob, p.pw2.bias);
         float* uc = u + row;
-        DuForEachAccGroup(trow + L::kColD, [&](int c0, const uint32_t (&v)[16]) {
-          uint32_t hi[16], lo[16];
-          float res[16];
+        if constexpr (unit == 2) {
+          DuAccToA(sh, trow, has_row, f_par, [&](int c0, const uint32_t (&v)[16], uint32_t (&hi)[16], uint32_t (&lo)[16]) {
+            float res[16];
 #pragma unroll
-          for (int j = 0; j < 16; ++j) res[j] = uc[(c0 + j) * LDU];                 // the residual: loads first, one exposed latency
+            for (int j = 0; j < 16; ++j) res[j] = uc[(c0 + j) * LDU];               // the residual: loads first, one exposed latency
 #pragma unroll
-          for (int j = 0; j < 16; ++j) {
-            const float val = __fadd_rn(__fadd_rn(__uint_as_float(v[j]), b2[c0 + j]), res[j]);
-            if (unit == 2) DuSplit(LeakyRelu(val), hi[j], lo[j]);
-            else uc[(c0 + j) * LDU] = val;
+            for (int j = 0; j < 16; ++j) DuSplit(LeakyRelu(__fadd_rn(__fadd_rn(__uint_as_float(v[j]), b2[c0 + j]), res[j])), hi[j], lo[j]);
+          });
+        } else {
+          if (has_row) {
+            DuForEachAccGroup(trow + L::kColD, [&](int c0, const uint32_t (&v)[16]) {
+              float res[16];
+#pragma unroll
+              for (int j = 0; j < 16; ++j) res[j] = uc[(c0 + j) * LDU];             // the residual: loads first, one exposed latency
+#pragma unroll
+              for (int j = 0; j < 16; ++j) uc[(c0 + j) * LDU] = __fadd_rn(__fadd_rn(__uint_as_float(v[j]), b2[c0 + j]), res[j]);
+            });
           }
-          if (unit == 2) {
-            lyra_tmem_st<16>(trow + L::kColAhi + (uint32_t)c0, hi);
-            lyra_tmem_st<16>(trow + L::kColAlo + (uint32_t)c0, lo);
-          }
-        });
+          row_sync();                                        // u' complete before anybody reads a neighbour's rows
+        }
       }
-      if (unit == 2) DuArriveA(sh);
-      else row_sync();                                       // u' complete before anybody reads a neighbour's rows
       LYRA_PHASE(3, ph);
     };
     unit_body(std::integral_constant<int, 0>());
